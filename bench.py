@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                 # our arm (one rank per GPU under torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path (oracle), rank 0 only
     python bench.py --config c3|c4|c5 ...                          # the other BASELINE.json configs (c2 = default)
+    python bench.py ... --dump-outputs DIR                         # + what the last timed step returned, as DIR/*.npy
 
 A step = one pass of the per-image pipeline over a batch of synthetic images: CLIP ViT-L/14-336 image tower on every
 512^2 crop + KL-VAE encoder / truncated decoder taps [unless --hot-path-only] -> implicit captioner -> UNet feature
@@ -61,10 +62,17 @@ def parse():
                          "(not a parity mode)")
     ap.add_argument("--vocab", default=None, choices=sorted(VOCABS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32 / "
+                         "float64, at most 64 MB in all): what ODISEEngine.infer() returned (c2 / c3 / c5), the MSDeformAttn "
+                         "and decoder outputs (c4), the CPU path's logits and inference maps (--impl reference); so that "
+                         "two builds can be compared output for output")
     ap.add_argument("--hot-path-only", action="store_true",
                     help="skip the KL-VAE (SURVEY.md 8f-1) and CLIP image tower (8f-2) stages: their taps / latent / "
                          "image embedding enter as synthetic tensors")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     c = CONFIGS[a.config]
     a.batch = a.batch or c["batch"]
     a.size = a.size or c["size"]
@@ -79,6 +87,33 @@ def peaks():
         return dict(bf16_burst=d["bf16_tflops"], bf16_sustained=d.get("bf16_tflops_sustained", d["bf16_tflops"]),
                     hbm=d["hbm_gbs"], source="measured")
     return dict(bf16_burst=1590.0, bf16_sustained=1400.0, hbm=6650.0, source="fallback")
+
+
+NPY_HEADER = 256                     # bytes an .npy header takes at most for the shapes written here
+
+
+def dump_outputs(arrays, out_dir, budget=64_000_000):
+    """Writes each array as out_dir/<name>.npy: float64 stays float64, other floating types and integers that float32
+    holds exactly become float32, larger integers float64.  The files, headers included, take at most `budget` bytes:
+    it is shared out smallest array first, and an array over its share is replaced by a fixed, seeded sample of its
+    flattened elements (the same indices on every run)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    conv = {}
+    for name, v in arrays.items():
+        v = v.detach().cpu()
+        if v.dtype == torch.bool:
+            v = v.to(torch.int32)
+        wide = v.dtype == torch.float64 or (not v.is_floating_point() and v.numel() > 0 and int(v.abs().max()) >= 2 ** 24)
+        conv[name] = v.to(torch.float64 if wide else torch.float32)
+    left = budget - NPY_HEADER * len(conv)
+    for i, (name, v) in enumerate(sorted(conv.items(), key=lambda kv: kv[1].numel() * kv[1].element_size())):
+        share = left // (len(conv) - i)
+        if v.numel() * v.element_size() > share:
+            g = torch.Generator().manual_seed(0)
+            v = v.flatten()[torch.randperm(v.numel(), generator=g)[:share // v.element_size()].sort().values]
+        left -= v.numel() * v.element_size()
+        np.save(os.path.join(out_dir, name + ".npy"), v.numpy())
 
 
 def n_crops(size):
@@ -198,9 +233,11 @@ class CpuHotPath:
         # odise.py:326-370: upsample to the input size, semantic + panoptic inference (instance inference is a top-k
         # over the same tensors; not timed on the CPU side)
         up = opp.upsample_masks(out["pred_masks"], (self.size, self.size))[0]
-        opp.semantic_inference(lg[0], up)
-        opp.panoptic_inference(lg[0], up, self.ncls, list(range(0, self.ncls, 2)))
+        sem = opp.semantic_inference(lg[0], up)
+        pan, segs = opp.panoptic_inference(lg[0], up, self.ncls, list(range(0, self.ncls, 2)))
         t_head = time.perf_counter() - t0
+        self.last = dict(pred_logits=lg[0], sem_seg=sem, panoptic_seg=pan, segments_info=torch.tensor(
+            [[s["id"], int(s["isthing"]), s["category_id"]] for s in segs], dtype=torch.int64).view(-1, 3))
         ips = 1.0 / (self.crops * t_unet + t_head)
         return dict(value=ips, unit="images/s", cores=self.n, kind="port",
                     sample=f"1 crop (512^2) through {'CLIP ViT-L/14 image tower + VAE enc + UNet + full VAE dec' if self.full else 'the UNet'} as the "
@@ -218,21 +255,20 @@ def run_reference(args):
                           "own CUDA kernel, oracle/_ref) is reported inside the c4 line of the `ours` arm"}), flush=True)
         return
     cpu = CpuHotPath(args.size, args.vocab, full=args.full)
-    t_start = time.perf_counter()
-    for _ in range(min(args.warmup, 1)):
+    for _ in range(args.warmup):
         cpu.sample()
     vals, info = [], None
     for _ in range(args.steps):
         info = cpu.sample()
         vals.append(info["value"])
-        if time.perf_counter() - t_start > 200:                 # keep the arm within a few minutes
-            break
+    if args.dump_outputs:
+        dump_outputs(cpu.last, args.dump_outputs)
     v = statistics.mean(vals)
     info["value"] = v
     ncls, npr = VOCABS[args.vocab]
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": v, "unit": "images/s", "n_gpus": args.gpus,
-        "steps": len(vals), "warmup": min(args.warmup, 1), "ms_per_step": 1000.0 / v, "higher_is_better": True,
+        "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1000.0 / v, "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": f"ODISE hot path, {args.size}x{args.size}, {args.vocab} ({npr} prompts), CPU oracle",
                    "baseline_config": args.config,
@@ -272,7 +308,8 @@ def run_c4(args, dev):
     ss = torch.as_tensor(shapes, dtype=torch.int64)
     lsi = torch.cat((ss.new_zeros(1), ss.prod(1).cumsum(0)[:-1]))
     value = torch.randn(N, S, M, D, generator=g).to(dev)
-    res = {}
+    res, dumps = {}, {}
+    reps, warm = args.steps, args.warmup
     for name, Lq in (("encoder_Lq=S", S), ("queries_Lq=256", 256)):
         ref_pts = torch.rand(N, Lq, L, 2, generator=g)
         offs = torch.randn(N, Lq, M, L, P, 2, generator=g) * 2.0
@@ -292,8 +329,9 @@ def run_c4(args, dev):
         def ours_fused():
             ops.msda_fused(value, dss, dls, dref, doffs, dlog, N, S, M, D, L, Lq, P, want_f32=False)
 
-        reps = 20 if Lq == S else 200
-        t_abi, t_fused = _time_ms(ours_abi, reps), _time_ms(ours_fused, reps)
+        t_abi = _time_ms(ours_abi, reps, warm)
+        dumps["msda_" + name.split("_")[0]] = out.clone()          # what the last timed odise_msda_forward_f32 wrote
+        t_fused = _time_ms(ours_fused, reps, warm)
         # what the gathers move through L1: 4 corners x 128 B per (query, head, sample)
         l1_bytes = 128.0 * 4 * N * Lq * M * L * P
         # compulsory bytes (SURVEY.md §8d): value once (at most what the samples can touch) + loc / attn (3 floats per
@@ -306,7 +344,7 @@ def run_c4(args, dev):
             from oracle import refmsda
             if refmsda.available():
                 ro = torch.empty_like(out)
-                t_ref = _time_ms(lambda: refmsda.forward(value, dss, dls, loc, aw, 128, out=ro), reps)
+                t_ref = _time_ms(lambda: refmsda.forward(value, dss, dls, loc, aw, 128, out=ro), reps, warm)
                 ours_abi()
                 torch.cuda.synchronize()
                 r.update(reference_kernel_us=1e3 * t_ref, reference_kernel_gbs=nbytes / t_ref / 1e6,
@@ -326,7 +364,13 @@ def run_c4(args, dev):
     c0 = lib.launch_count()
     he.transformer_decoder(pd, N)
     launches = lib.launch_count() - c0
-    t_dec = _time_ms(lambda: he.transformer_decoder(pd, N), 10)
+    last = {}
+
+    def dec_step():
+        last["heads"] = he.transformer_decoder(pd, N)
+
+    t_dec = _time_ms(dec_step, reps, warm)
+    dumps.update({"decoder_" + k: v for k, v in last["heads"][-1].items()})      # the last prediction head
     HW = (args.size // 4) ** 2
     plane = 4.0                                     # bytes per element of a (hi, lo) bf16 operand pair
     # K and V^T planes (head-padded 8 x 64 columns) of every layer, read once by its cross-attention
@@ -342,7 +386,7 @@ def run_c4(args, dev):
     enc = res["encoder_Lq=S"]
     line = {
         "metric": "MSDeformAttn + masked-attention decoder microbench, 256 queries x 4 scales, HBM GB/s",
-        "value": enc["ours_abi_gbs"], "unit": "GB/s", "n_gpus": 1, "steps": 20, "warmup": 3,
+        "value": enc["ours_abi_gbs"], "unit": "GB/s", "n_gpus": 1, "steps": reps, "warmup": warm,
         "ms_per_step": enc["ours_abi_us"] / 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "f32", "data": "synthetic",
         "config": {"workload": f"c4: MSDeformAttn forward, N={N}, 4 levels {shapes}, S={S}, M=8, D=32, P=4 (value = compulsory "
@@ -355,6 +399,8 @@ def run_c4(args, dev):
         "c4": res,
         "gpu_launches": int(launches),
     }
+    if args.dump_outputs:
+        dump_outputs(dumps, args.dump_outputs)
     print(json.dumps(line), flush=True)
 
 
@@ -419,10 +465,13 @@ def main():
         graph.replay()
         gather_logits(out["pred_logits"])
 
+    last = {}
+
     def e2e_step():
         r = eng.infer(images, outputs="panoptic")
         if world > 1:
             gather_logits(out["pred_logits"])
+        last["r"] = r
         return r
 
     for _ in range(args.warmup):
@@ -435,6 +484,9 @@ def main():
         e2e_step()
     ms_e2e = timed(e2e_step, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # infer() returns its pinned host buffers, which the next call overwrites: write them before anything else runs
+        dump_outputs(last["r"], args.dump_outputs)
 
     # roofline of the dominant kernel (gemm_tc_kernel): one eager pass with per-launch CUDA events
     lib.profile_begin()

@@ -2,9 +2,36 @@
 the REFERENCE's own code on them in the build container (/root/reference present) and commits the outputs under
 tests/golden/ref_*.pt, and by tests/test_golden_cpu.py, which replays the oracle on the same inputs wherever the suite
 runs (the GPU box has no /root/reference)."""
+import contextlib
+
 import torch
 
 from odise_b200 import spec
+
+# torch splits CPU reductions (convolutions, GEMMs, norms) over its intra-op threads, so the bits of a result depend on
+# the thread count.  The golden files were written with this many threads; comparisons that must be bit-exact run with
+# the same count (whatever the machine's core count).
+GOLDEN_THREADS = 8
+
+
+@contextlib.contextmanager
+def golden_threads():
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(n)
+
+
+def sample(t, n=1024, seed=0):
+    """A fixed, seeded sample of n elements of t, flattened (all of t when it has at most n): golden files keep this
+    instead of a whole large tensor, and the tests take the same sample of what they compute."""
+    flat = t.reshape(-1)
+    if flat.numel() <= n:
+        return flat.clone()
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(seed))[:n]
+    return flat[idx.to(flat.device)]
 
 
 def head_case():

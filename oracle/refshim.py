@@ -1,7 +1,7 @@
 """Import scaffolding that lets the REFERENCE's own Python (vendored Mask2Former + odise/modeling/meta_arch/odise.py)
-run on CPU in the build container, where detectron2 / fvcore / open_clip / ldm / ... are not installed.
-TEST INFRASTRUCTURE ONLY — used by tools/make_golden_*.py and by CPU tests that are skipped when /root/reference
-is absent (it never exists on the GPU box).  The arithmetic executed is the reference's; only third-party
+run on CPU where detectron2 / fvcore / open_clip / ldm / ... are not installed.
+TEST INFRASTRUCTURE ONLY — used by tools/make_golden_ref.py and tools/make_golden_pins.py, which store what the
+reference computes under tests/golden/; no test imports it.  The arithmetic executed is the reference's; only third-party
 registry / config decorators and the tiny detectron2 layer helpers are stubbed (SURVEY.md Appendix C):
 
   detectron2.layers.Conv2d     = nn.Conv2d with optional .norm / .activation applied in forward  (d2 wrappers.py)
@@ -164,6 +164,25 @@ def install():
     pkg("odise.utils", os.path.join(REF, "odise", "utils"))
     pkg("odise.checkpoint", os.path.join(REF, "odise", "checkpoint"))
     _installed = True
+
+
+def ref_head(m):
+    """The reference's pixel decoder and ODISE decoder (m = modules()) in the configuration of the label model."""
+    S = m.ShapeSpec
+    shape = {f"s{i}": S(channels=512, stride=2 ** i) for i in (2, 3, 4, 5)}
+    pd = m.MSDeformAttnPixelDecoder(shape, transformer_dropout=0.0, transformer_nheads=8,
+                                    transformer_dim_feedforward=1024, transformer_enc_layers=6, conv_dim=256,
+                                    mask_dim=256, norm="GN", transformer_in_features=["s3", "s4", "s5"],
+                                    common_stride=4).eval()
+    dec = m.ODISEMultiScaleMaskedTransformerDecoder(
+        class_embed=m.PseudoClassEmbed(133), post_mask_embed=m.PooledMaskEmbed(256, 256, 256), in_channels=256,
+        mask_classification=True, num_classes=133, hidden_dim=256, num_queries=100, nheads=8, dim_feedforward=2048,
+        dec_layers=9, pre_norm=False, enforce_input_project=False, mask_dim=256).eval()
+    return pd, dec
+
+
+def strip(sd, prefix):
+    return {k[len(prefix):]: v for k, v in sd.items() if k.startswith(prefix)}
 
 
 def modules():

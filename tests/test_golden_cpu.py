@@ -68,9 +68,11 @@ def test_postprocess_matches_reference_golden():
 def test_ldm_drivers_match_reference_golden():
     ref = _load("ref_ldm_driver.pt")
     d = cases.ldm_case()
-    for a, b in zip(oldm.unet_features(d["unet"], d["x"], d["ctx"], d["cond"]), ref["unet_feats"]):
+    with cases.golden_threads():                       # bit-exact: same reduction order as when the file was written
+        feats = oldm.unet_features(d["unet"], d["x"], d["ctx"], d["cond"])
+        lat, ef = oldm.encoder_features(d["vae"], d["img"])
+        df = oldm.decoder_features(d["vae"], ref["latent"])
+    for a, b in zip(feats, ref["unet_feats"]):
         assert torch.equal(a, b)
-    lat, ef = oldm.encoder_features(d["vae"], d["img"])
     assert torch.equal(lat, ref["latent"]) and all(torch.equal(a, b) for a, b in zip(ef, ref["enc_feats"]))
-    df = oldm.decoder_features(d["vae"], ref["latent"])
     assert len(df) == 2 and all(torch.equal(a, b) for a, b in zip(df, ref["dec_feats"]))

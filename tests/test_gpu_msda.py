@@ -69,21 +69,29 @@ def test_msda_fused_vs_oracle(cuda):
         assert (pl.float().view(N, S, -1).cpu() - want).abs().max().item() < 1e-4 * max(1.0, want.abs().max().item())
 
 
+REFKERNEL_CASES = (dict(seed=4, N=2, M=8, D=32, shapes=[(16, 16), (32, 32), (64, 64)], Lq=5376, P=4, spread=1.5),
+                   dict(seed=8, N=2, M=8, D=32, shapes=[(16, 16), (32, 32), (64, 64), (128, 128)], Lq=300, P=4, spread=1.4),
+                   dict(seed=6, N=3, M=4, D=64, shapes=[(7, 5), (3, 9)], Lq=11, P=3, spread=2.0))
+
+
 def test_msda_vs_reference_kernel(cuda):
-    """Same inputs through the REFERENCE's own CUDA kernel compiled for sm_100a (oracle/_ref/libref_msda.so, built from
-    ops/src/cuda/ms_deform_im2col_cuda.cuh by oracle/Makefile): fp32, only the summation order differs."""
+    """Same inputs as the REFERENCE's own CUDA kernel compiled for sm_100a (ops/src/cuda/ms_deform_im2col_cuda.cuh behind
+    oracle/ref_msda_host.cu) was given by tools/make_golden_refkernel.py, which stored a fixed sample of its outputs and
+    the sum of every output row in tests/golden/refkernel_msda.pt: fp32, only the summation order differs.  A row sum
+    holds M x D elements, so its bound is M x D times the element bound."""
     from odise_b200 import lib
-    from oracle import refmsda
-    if not refmsda.available():
-        pytest.skip("oracle/_ref/libref_msda.so not built (needs /root/reference at build time)")
-    for cfg in (dict(seed=4, N=2, M=8, D=32, shapes=[(16, 16), (32, 32), (64, 64)], Lq=5376, P=4, spread=1.5),
-                dict(seed=8, N=2, M=8, D=32, shapes=[(16, 16), (32, 32), (64, 64), (128, 128)], Lq=300, P=4, spread=1.4),
-                dict(seed=6, N=3, M=4, D=64, shapes=[(7, 5), (3, 9)], Lq=11, P=3, spread=2.0)):
+    from oracle import cases
+    gold = torch.load(os.path.join(GOLD, "refkernel_msda.pt"), weights_only=True)
+    assert len(gold["samples"]) == len(REFKERNEL_CASES)
+    for cfg, want, rows, amax in zip(REFKERNEL_CASES, gold["samples"], gold["row_sums"], gold["absmax"]):
         value, ss, lsi, loc, aw = (t.to(cuda) for t in _problem(**cfg))
-        want = refmsda.forward(value, ss, lsi, loc, aw, 128)
         got = lib.msda_forward(value, ss, lsi, loc, aw, 128)
         torch.cuda.synchronize()
-        assert (got - want).abs().max().item() < 1e-5 * max(1.0, want.abs().max().item())
+        assert abs(got.abs().max().item() - amax) < 1e-5 * max(1.0, amax)
+        tol = 1e-5 * max(1.0, amax)
+        assert (cases.sample(got, want.numel()).cpu() - want).abs().max().item() < tol
+        assert rows.shape == got.shape[:-1]
+        assert (got.double().sum(-1).cpu() - rows.double()).abs().max().item() < tol * got.shape[-1]
 
 
 def test_msda_golden(cuda):

@@ -1,16 +1,18 @@
-"""CPU tests that PIN the oracle (oracle/) against the reference's own code imported from /root/reference
-(skipped where that tree is absent, i.e. on the GPU box) and check the parameter inventory of odise_b200/spec.py."""
+"""CPU tests that PIN the oracle (oracle/) against the reference's own code, and check the parameter inventory of
+odise_b200/spec.py.  What the reference computed on these tests' inputs (see the *_inputs functions) is stored in
+tests/golden/ref_pins.pt by tools/make_golden_pins.py, so the tests need no reference tree."""
 import os
-import types
 
-import pytest
 import torch
 
 from odise_b200 import spec
+from oracle import cases
 from oracle import ldm as oldm
-from oracle import m2f, refshim
+from oracle import m2f
 
-needs_ref = pytest.mark.skipif(not refshim.available(), reason="/root/reference not present")
+
+def _pins():
+    return torch.load(os.path.join(os.path.dirname(__file__), "golden", "ref_pins.pt"), weights_only=True)
 
 
 def _shapes(params, prefix):
@@ -38,115 +40,88 @@ def _head_sd(seed=0):
     return spec.synth_state_dict(spec.head_params(), seed)
 
 
-@needs_ref
 def test_head_inventory_matches_reference_modules():
-    m = refshim.modules()
-    pd, dec = _ref_head(m)
-    want = {**{"sem_seg_head.pixel_decoder." + k: tuple(v.shape) for k, v in pd.state_dict().items()},
-            **{"sem_seg_head.predictor." + k: tuple(v.shape) for k, v in dec.state_dict().items()}}
     got = {n: tuple(s) for n, s, _ in spec.pixel_decoder_params() + spec.decoder_params()}
-    assert got == want
+    assert got == _pins()["head_state_shapes"]
 
 
-def _ref_head(m):
-    S = m.ShapeSpec
-    shape = {f"s{i}": S(channels=512, stride=2 ** i) for i in (2, 3, 4, 5)}
-    pd = m.MSDeformAttnPixelDecoder(shape, transformer_dropout=0.0, transformer_nheads=8,
-                                    transformer_dim_feedforward=1024, transformer_enc_layers=6, conv_dim=256,
-                                    mask_dim=256, norm="GN", transformer_in_features=["s3", "s4", "s5"],
-                                    common_stride=4).eval()
-    dec = m.ODISEMultiScaleMaskedTransformerDecoder(
-        class_embed=m.PseudoClassEmbed(133), post_mask_embed=m.PooledMaskEmbed(256, 256, 256), in_channels=256,
-        mask_classification=True, num_classes=133, hidden_dim=256, num_queries=100, nheads=8, dim_feedforward=2048,
-        dec_layers=9, pre_norm=False, enforce_input_project=False, mask_dim=256).eval()
-    return pd, dec
-
-
-def _strip(sd, prefix):
-    return {k[len(prefix):]: v for k, v in sd.items() if k.startswith(prefix)}
-
-
-@needs_ref
-@torch.no_grad()
-def test_head_oracle_equals_reference():
-    m = refshim.modules()
-    pd, dec = _ref_head(m)
+def head_inputs():
+    """Seeded inputs of the head check: weights, backbone features for the pixel decoder, inputs of the decoder (drawn
+    on their own, so the decoder check does not ride on the pixel decoder's rounding: its mask thresholds make it
+    discontinuous) and of the scoring."""
     sd = _head_sd(1)
-    pd.load_state_dict(_strip(sd, "sem_seg_head.pixel_decoder."))
-    dec.load_state_dict(_strip(sd, "sem_seg_head.predictor."))
     g = torch.Generator().manual_seed(5)
     feats = {f"s{i}": torch.randn(2, 512, 128 // 2 ** i, 128 // 2 ** i, generator=g) for i in (2, 3, 4, 5)}
-    mf_r, t_r, ms_r = pd.forward_features(feats)
-    mf_o, t_o, ms_o = m2f.pixel_decoder(sd, feats, "sem_seg_head.pixel_decoder.")
-    assert torch.allclose(mf_o, mf_r, rtol=1e-4, atol=1e-5)
-    for a, b in zip(ms_o, ms_r):
-        assert torch.allclose(a, b, rtol=1e-4, atol=1e-5)
-    out_r = dec(ms_r, mf_r)
-    out_o, _ = m2f.transformer_decoder(sd, ms_r, mf_r, "sem_seg_head.predictor.")
-    for k in ("pred_masks", "mask_embed", "mask_pooled_features"):
-        assert torch.allclose(out_o[k], out_r[k], rtol=1e-3, atol=1e-4), k
-    assert torch.equal(out_o["logit_scale"], out_r["logit_scale"])
-    for a, b in zip(out_o["aux_outputs"], out_r["aux_outputs"]):
-        assert torch.allclose(a["pred_masks"], b["pred_masks"], rtol=1e-3, atol=1e-4)
-    # scoring: CategoryODISE.cal_pred_logits on the reference class itself
+    ms = [torch.randn(2, 256, 128 // s, 128 // s, generator=g) for s in (32, 16, 8)]
+    mf = torch.randn(2, 256, 32, 32, generator=g)
     sizes = [1, 3, 2, 1, 4] * 4
+    me = torch.randn(2, 100, 256, generator=g)
     te = torch.randn(sum(sizes), 256, generator=g)
     ne = torch.randn(1, 256, generator=g)
-    labels = [["x"] * n for n in sizes]
-    ref = m.CategoryODISE.cal_pred_logits(None, dict(mask_embed=out_r["mask_embed"], text_embed=te, null_embed=ne,
-                                                     labels=labels, logit_scale=out_r["logit_scale"]))
-    mine = m2f.cal_pred_logits(out_r["mask_embed"], te, ne, out_r["logit_scale"], sizes)
-    assert torch.allclose(mine, ref, rtol=1e-5, atol=1e-5)
+    return sd, feats, (ms, mf), (me, te, ne, sizes)
 
 
-@needs_ref
+def _close(a, b, rtol, atol):
+    a = cases.sample(a, b.numel())
+    assert a.shape == b.shape and torch.allclose(a, b, rtol=rtol, atol=atol), (a - b).abs().max().item()
+
+
+@torch.no_grad()
+def test_head_oracle_equals_reference():
+    """Pixel decoder, decoder and CategoryODISE.cal_pred_logits against the reference's outputs (fixed samples)."""
+    ref = _pins()["head"]
+    sd, feats, (ms, mf), (me, te, ne, sizes) = head_inputs()
+    mf_o, t_o, ms_o = m2f.pixel_decoder(sd, feats, "sem_seg_head.pixel_decoder.")
+    _close(mf_o, ref["mask_features"], 1e-4, 1e-5)
+    assert len(ms_o) == len(ref["multi_scale"])
+    for a, b in zip(ms_o, ref["multi_scale"]):
+        _close(a, b, 1e-4, 1e-5)
+    out_o, _ = m2f.transformer_decoder(sd, ms, mf, "sem_seg_head.predictor.")
+    for k in ("pred_masks", "mask_embed", "mask_pooled_features"):
+        _close(out_o[k], ref[k], 1e-3, 1e-4)
+    assert torch.equal(out_o["logit_scale"], ref["logit_scale"])
+    assert len(out_o["aux_outputs"]) == len(ref["aux_pred_masks"])
+    for a, b in zip(out_o["aux_outputs"], ref["aux_pred_masks"]):
+        _close(a["pred_masks"], b, 1e-3, 1e-4)
+    mine = m2f.cal_pred_logits(me, te, ne, out_o["logit_scale"], sizes)
+    assert torch.allclose(mine, ref["pred_logits"], rtol=1e-5, atol=1e-5)
+
+
 @torch.no_grad()
 def test_position_embedding_and_msdeformattn_equal_reference():
-    m = refshim.modules()
-    x = torch.zeros(2, 256, 7, 9)
-    assert torch.allclose(m2f.position_embedding_sine(2, 7, 9), m.PositionEmbeddingSine(128, normalize=True)(x), atol=1e-6)
+    _close(m2f.position_embedding_sine(2, 7, 9), _pins()["position_embedding"], 0, 1e-6)
 
 
-@needs_ref
-@torch.no_grad()
-def test_reference_ldm_driver_runs_on_oracle_unet():
-    """The reference's LdmExtractor.unet_forward / encoder_forward / decoder_forward (ldm.py:424-533) executed
-    VERBATIM on the oracle modules == oracle.ldm.unet_features / encoder_features / decoder_features."""
-    import importlib
-    refshim.install()
-    rl = importlib.import_module("odise.modeling.meta_arch.ldm")
-    rl.timestep_embedding = oldm.timestep_embedding
-    rl.DiagonalGaussianDistribution = oldm.DiagonalGaussianDistribution
+def ldm_driver_inputs():
     torch.manual_seed(0)
     unet = oldm.UNetModel(model_channels=64, num_heads=8, context_dim=48).eval()
     for p in unet.parameters():
         torch.nn.init.normal_(p, std=0.05)
     x, ctx = torch.randn(2, 4, 16, 16), torch.randn(2, 5, 48)
     cond = torch.randn(2, 256)
-    fake = types.SimpleNamespace(ldm=types.SimpleNamespace(unet=unet),
-                                 unet_blocks=[unet.output_blocks[i] for i in oldm.UNET_TAP_BLOCKS])
-    _, ref_feats = rl.LdmExtractor.unet_forward(fake, x, torch.zeros(2, dtype=torch.long), ctx, cond_emb=cond.clone())
-    mine = oldm.unet_features(unet, x, ctx, cond)
-    assert len(ref_feats) == 4
-    for a, b in zip(mine, ref_feats):
-        assert torch.equal(a, b)
     vae = oldm.AutoencoderKL().eval()
-    enc_blocks = [vae.encoder.down[i].block[j] for i in range(4) for j in range(2)]
-    dec_blocks = [vae.decoder.up[i].block[j] for i in reversed(range(4)) for j in range(3)]
-    fake = types.SimpleNamespace(
-        ldm=types.SimpleNamespace(encoder=vae.encoder, decoder=vae.decoder,
-                                  ldm=types.SimpleNamespace(first_stage_model=vae, scale_factor=oldm.SCALE_FACTOR)),
-        encoder_blocks=[enc_blocks[i] for i in oldm.ENC_TAP_BLOCKS],
-        decoder_blocks=[dec_blocks[i] for i in oldm.DEC_TAP_BLOCKS])
-    fake.encoder_forward = lambda im: rl.LdmExtractor.encoder_forward(fake, im)
-    fake.decoder_forward = lambda z: rl.LdmExtractor.decoder_forward(fake, z)
     img = torch.randn(1, 3, 64, 64)
-    lat_r, ef_r = rl.LdmExtractor.encode_to_latent(fake, img)
-    lat_o, ef_o = oldm.encoder_features(vae, img)
-    assert torch.equal(lat_r, lat_o) and all(torch.equal(a, b) for a, b in zip(ef_r, ef_o))
-    _, df_r = rl.LdmExtractor.decode_to_image(fake, lat_r)
-    df_o = oldm.decoder_features(vae, lat_o)
-    assert len(df_r) == 2 and all(torch.equal(a, b) for a, b in zip(df_r, df_o))
+    return unet, x, ctx, cond, vae, img
+
+
+@torch.no_grad()
+def test_reference_ldm_driver_runs_on_oracle_unet():
+    """The reference's LdmExtractor.unet_forward / encoder_forward / decoder_forward (ldm.py:424-533) executed
+    VERBATIM on the oracle modules == oracle.ldm.unet_features / encoder_features / decoder_features (fixed samples)."""
+    ref = _pins()["ldm_driver"]
+    unet, x, ctx, cond, vae, img = ldm_driver_inputs()
+    with cases.golden_threads():                       # bit-exact: same reduction order as when the file was written
+        mine = oldm.unet_features(unet, x, ctx, cond)
+        lat_o, ef_o = oldm.encoder_features(vae, img)
+        df_o = oldm.decoder_features(vae, lat_o)
+    assert len(mine) == len(ref["unet_feats"]) == 4
+    for a, b in zip(mine, ref["unet_feats"]):
+        assert torch.equal(cases.sample(a, b.numel()), b)
+    assert len(ef_o) == len(ref["enc_feats"])
+    assert torch.equal(cases.sample(lat_o, ref["latent"].numel()), ref["latent"])
+    assert all(torch.equal(cases.sample(a, b.numel()), b) for a, b in zip(ef_o, ref["enc_feats"]))
+    assert len(df_o) == len(ref["dec_feats"]) == 2
+    assert all(torch.equal(cases.sample(a, b.numel()), b) for a, b in zip(df_o, ref["dec_feats"]))
 
 
 def test_q_sample_constants():
@@ -154,33 +129,6 @@ def test_q_sample_constants():
     assert abs(a - 0.999575) < 1e-6 and abs(b - 0.029155) < 1e-6   # SURVEY.md §8a row a6
     n = oldm.shared_noise()
     assert n.shape == (1, 4, 64, 64)
-
-
-@needs_ref
-@torch.no_grad()
-def test_postprocess_oracle_equals_reference_methods():
-    """oracle/postprocess.py vs the reference's MaskFormer.semantic_inference / panoptic_inference
-    (maskformer_model.py:280-342) called on a fake self through the shim."""
-    import importlib
-    from oracle import postprocess as opp
-    refshim.install()
-    MF = importlib.import_module("mask2former.maskformer_model").MaskFormer
-    g = torch.Generator().manual_seed(4)
-    Q, K, H, W = 30, 9, 40, 56
-    cls = torch.randn(Q, K + 1, generator=g) * 3
-    cls[:, -1] -= 2
-    yy, xx = torch.meshgrid(torch.arange(H).float(), torch.arange(W).float(), indexing="ij")
-    pred = torch.stack([(6 + 10 * torch.rand(1, generator=g) - ((yy - torch.rand(1, generator=g) * H) ** 2 +
-                                                               (xx - torch.rand(1, generator=g) * W) ** 2).sqrt()) * 2
-                        for _ in range(Q)])
-    things = [0, 2, 4]
-    fake = types.SimpleNamespace(sem_seg_head=types.SimpleNamespace(num_classes=K), object_mask_threshold=0.0,
-                                 overlap_threshold=0.8, num_queries=Q, test_topk_per_image=10, panoptic_on=True,
-                                 metadata=types.SimpleNamespace(thing_dataset_id_to_contiguous_id={i: t for i, t in enumerate(things)}))
-    assert torch.equal(MF.semantic_inference(fake, cls, pred), opp.semantic_inference(cls, pred))
-    pr, ir = MF.panoptic_inference(fake, cls, pred)
-    po, io = opp.panoptic_inference(cls, pred, K, things)
-    assert torch.equal(pr, po) and ir == io and len(ir) > 0
 
 
 def test_clip_inventory_matches_oracle_module():
@@ -192,34 +140,26 @@ def test_clip_inventory_matches_oracle_module():
     assert 303e6 < sum(torch.Size(s).numel() for s in got.values()) < 305e6      # ViT-L/14-336 image tower
 
 
-@needs_ref
-@torch.no_grad()
-def test_reference_clip_glue_runs_on_oracle_visual():
-    """ClipAdapter._encode_image (clip.py:177-222) executed verbatim on the oracle VisionTransformer == oracle.encode_image."""
-    import importlib
+def clip_glue_inputs():
     from oracle import clip as oclip
-    refshim.install()
-    rc = importlib.import_module("odise.modeling.meta_arch.clip")
-    import einops
-    rc.rearrange = einops.rearrange
     torch.manual_seed(0)
     v = oclip.VisionTransformer(image_size=56, patch=14, width=64, layers=2, heads=4, out_dim=32).eval()
     for p in v.parameters():
         torch.nn.init.normal_(p, std=0.1)
-    img = torch.randn(2, 3, 56, 56)
-    fake = types.SimpleNamespace(clip=types.SimpleNamespace(visual=v))
-    emb_ref, _ = rc.ClipAdapter._encode_image(fake, img)
+    return v, torch.randn(2, 3, 56, 56)
+
+
+@torch.no_grad()
+def test_reference_clip_glue_runs_on_oracle_visual():
+    """ClipAdapter._encode_image (clip.py:177-222) executed verbatim on the oracle VisionTransformer == oracle.encode_image."""
+    from oracle import clip as oclip
+    v, img = clip_glue_inputs()
+    emb_ref = _pins()["clip_image_embed"]
     assert torch.allclose(emb_ref, oclip.encode_image(v, img), rtol=1e-5, atol=1e-6)
 
 
-@needs_ref
-@torch.no_grad()
-def test_reference_maskclip_runs_on_oracle_visual():
-    """MaskCLIP.get_mask_embed / pred_logits (clip.py:252-351) executed verbatim on the oracle VisionTransformer."""
-    import importlib
+def maskclip_inputs():
     from oracle import clip as oclip
-    refshim.install()
-    rc = importlib.import_module("odise.modeling.meta_arch.clip")
     torch.manual_seed(1)
     v = oclip.VisionTransformer(image_size=56, patch=14, width=128, layers=2, heads=2, out_dim=32).eval()
     for p in v.parameters():
@@ -227,41 +167,41 @@ def test_reference_maskclip_runs_on_oracle_visual():
     img = torch.rand(2, 3, 96, 96)
     masks = torch.randn(2, 5, 24, 24) * 3
     masks[0, 0] = -5.0                                         # a query whose mask touches no patch at all
-    fake = types.SimpleNamespace(clip=types.SimpleNamespace(visual=v), image_size=(56, 56),
-                                 clip_preprocess=lambda im: oclip.preprocess(im, 56), logit_scale=torch.tensor(37.0))
-    fake._mask_clip_forward = lambda *a: rc.MaskCLIP._mask_clip_forward(fake, *a)
-    fake.encode_image_with_mask = lambda *a: rc.MaskCLIP.encode_image_with_mask(fake, *a)
-    ref = rc.MaskCLIP.get_mask_embed(fake, img, masks)
-    got = oclip.get_mask_embed(v, img, masks)
-    assert ref.shape == (2, 5, 32) and torch.allclose(ref, got, rtol=1e-5, atol=1e-6)
     text = torch.randn(7, 32)
     labels = [["a", "b"], ["c"], ["d", "e", "f"], ["g"]]
-    lr = rc.MaskCLIP.pred_logits(fake, ref, text, labels)
-    lo = oclip.maskclip_pred_logits(got, text, [len(l) for l in labels], fake.logit_scale)
-    assert torch.allclose(lr, lo, rtol=1e-5, atol=1e-5)
+    return v, img, masks, text, labels
 
 
-@needs_ref
 @torch.no_grad()
-def test_reference_pooling_clip_head_ensemble():
-    """PoolingCLIPHead.forward (odise.py:1469-1542) run verbatim with a stubbed MaskCLIP == oracle ensemble."""
+def test_reference_maskclip_runs_on_oracle_visual():
+    """MaskCLIP.get_mask_embed / pred_logits (clip.py:252-351, logit scale 37) executed verbatim on the oracle
+    VisionTransformer."""
     from oracle import clip as oclip
-    refshim.install()
-    import importlib
-    ro = importlib.import_module("odise.modeling.meta_arch.odise")
+    v, img, masks, text, labels = maskclip_inputs()
+    ref = _pins()["maskclip"]
+    got = oclip.get_mask_embed(v, img, masks)
+    assert ref["mask_embed"].shape == (2, 5, 32) and torch.allclose(ref["mask_embed"], got, rtol=1e-5, atol=1e-6)
+    lo = oclip.maskclip_pred_logits(got, text, [len(l) for l in labels], torch.tensor(37.0))
+    assert torch.allclose(ref["logits"], lo, rtol=1e-5, atol=1e-5)
+
+
+def ensemble_inputs():
     torch.manual_seed(2)
     test_labels = [["cat", "kitty"], ["unicorn"], ["dog"], ["spaceship", "rocket"]]
     train_labels = [["cat"], ["dog", "puppy"], ["tree"]]
     cat_logits, clip_logits = torch.randn(2, 6, 4) * 4, torch.randn(2, 6, 4) * 4
-    fake = types.SimpleNamespace(training=False, test_labels=test_labels, train_labels=train_labels, prompt="photo",
-                                 with_bg=False, bg_labels=None, alpha=0.3, beta=0.7, normalize_logits=True,
-                                 get_and_cache_test_text_embed=lambda labels: None,
-                                 clip=lambda im, m, t, l: {"mask_pred_open_logits": clip_logits})
-    out = ro.PoolingCLIPHead.forward(fake, {"pred_open_logits": cat_logits.clone(), "images": torch.zeros(1),
-                                            "pred_masks": None})
+    return test_labels, train_labels, cat_logits, clip_logits
+
+
+@torch.no_grad()
+def test_reference_pooling_clip_head_ensemble():
+    """PoolingCLIPHead.forward (odise.py:1469-1542, alpha 0.3, beta 0.7, prompt "photo") run verbatim with a stubbed
+    MaskCLIP == oracle ensemble."""
+    from oracle import clip as oclip
+    test_labels, train_labels, cat_logits, clip_logits = ensemble_inputs()
     ov = torch.tensor([1, 0, 1, 0])
     got = oclip.pooling_clip_ensemble(cat_logits, clip_logits, ov, 0.3, 0.7)
-    assert torch.allclose(out["pred_open_logits"], got, rtol=1e-6, atol=1e-6)
+    assert torch.allclose(_pins()["ensemble"], got, rtol=1e-6, atol=1e-6)
     full = torch.randn(2, 6, 5)
     merged = oclip.merge_with_void(full, got)
     assert torch.allclose(merged.exp().sum(-1), torch.ones(2, 6) + 5e-8, atol=1e-5)
@@ -281,53 +221,52 @@ def test_clip_text_inventory_matches_oracle_module():
     assert missing == {"text_projection", "logit_scale"} and not (set(conv) - set(small.state_dict()))
 
 
-@needs_ref
-@torch.no_grad()
-def test_reference_encode_text_runs_on_oracle_text_tower():
-    """ClipAdapter._encode_text (clip.py:138-152) executed verbatim on the oracle TextTransformer == oracle.encode_text."""
-    import importlib
+def encode_text_inputs():
     from oracle import clip as oclip
-    refshim.install()
-    rc = importlib.import_module("odise.modeling.meta_arch.clip")
     torch.manual_seed(3)
     m = oclip.TextTransformer(vocab=50, ctx=9, width=64, layers=2, heads=2, out_dim=32).eval()
     for p in m.parameters():
         torch.nn.init.normal_(p, std=0.1)
     ids = torch.randint(1, 40, (3, 9))
     ids[0, 4], ids[1, 8], ids[2, 2] = 49, 49, 49                          # EOT = highest id
-    fake = types.SimpleNamespace(clip=m)
-    emb_ref, enc_ref = rc.ClipAdapter._encode_text(fake, ids)
+    return m, ids
+
+
+@torch.no_grad()
+def test_reference_encode_text_runs_on_oracle_text_tower():
+    """ClipAdapter._encode_text (clip.py:138-152) executed verbatim on the oracle TextTransformer == oracle.encode_text."""
+    from oracle import clip as oclip
+    m, ids = encode_text_inputs()
+    ref = _pins()["text_tower"]
+    emb_ref, enc_ref = ref["embed"], ref["encodings"]
     emb, enc = oclip.encode_text(m, ids)
     assert torch.allclose(emb_ref, emb, rtol=1e-5, atol=1e-6) and torch.allclose(enc_ref, enc, rtol=1e-5, atol=1e-6)
 
 
-@needs_ref
 def test_plugin_surface_matches_reference_modules():
     """SURVEY §8b B-1 / B-2: the B200 plugin classes take the constructor keywords the LazyConfigs pass
     (configs/common/models/odise_with_label.py:16-29, mask_generator_with_label.py:29-66) and expect exactly the state-dict
     keys of the reference modules they replace."""
     import inspect
     from odise_b200 import plugin
-    m = refshim.modules()
-    pd, dec = _ref_head(m)
+    pins = _pins()
     head = plugin.B200MaskFormerHead(num_classes=133, device="cpu")
-    want = {"pixel_decoder." + k for k in pd.state_dict()} | {"predictor." + k for k in dec.state_dict()}
+    want = {k[len("sem_seg_head."):] for k in pins["head_state_shapes"]}
     assert set(head.expected_keys()) == want
-    for mine, ref in ((plugin.B200MSDeformAttnPixelDecoder, m.MSDeformAttnPixelDecoder),
-                      (plugin.B200ODISEMultiScaleMaskedTransformerDecoder, m.ODISEMultiScaleMaskedTransformerDecoder),
-                      (plugin.B200PooledMaskEmbed, m.PooledMaskEmbed), (plugin.B200PseudoClassEmbed, m.PseudoClassEmbed)):
-        ref_kw = [p for c in ref.__mro__ if c.__module__.startswith(("odise", "mask2former"))
-                  for p in inspect.signature(c.__init__).parameters if p not in ("self", "kwargs", "args")]
+    for mine, ref in ((plugin.B200MSDeformAttnPixelDecoder, "MSDeformAttnPixelDecoder"),
+                      (plugin.B200ODISEMultiScaleMaskedTransformerDecoder, "ODISEMultiScaleMaskedTransformerDecoder"),
+                      (plugin.B200PooledMaskEmbed, "PooledMaskEmbed"), (plugin.B200PseudoClassEmbed, "PseudoClassEmbed")):
+        ref_kw = pins["constructor_keywords"][ref]
         mine_kw = set(inspect.signature(mine.__init__).parameters)
         assert set(ref_kw) <= mine_kw, (mine.__name__, set(ref_kw) - mine_kw)
-    # the two config files' keyword sets, parsed from the files themselves
-    cfg = open(os.path.join(refshim.REF, "configs/common/models/odise_with_label.py")).read()
+    # the keywords the label model's config passes (odise_with_label.py), as read from the file
+    cfg = set(pins["odise_with_label_keywords"])
     bb_kw = {"feature_extractor", "out_features", "use_checkpoint", "slide_training"}
-    assert all(k + "=" in cfg for k in bb_kw)
+    assert bb_kw <= cfg
     assert bb_kw <= set(inspect.signature(plugin.B200FeatureExtractorBackbone.__init__).parameters)
     fe_kw = {"encoder_block_indices", "unet_block_indices", "decoder_block_indices", "steps", "learnable_time_embed",
              "num_timesteps", "clip_model_name"}
-    assert all(k + "=" in cfg for k in fe_kw)
+    assert fe_kw <= cfg
     assert fe_kw <= set(inspect.signature(plugin.B200LdmImplicitCaptionerExtractor.__init__).parameters)
     fe = plugin.B200LdmImplicitCaptionerExtractor(frozen_state_dict={}, device="cpu")
     bb = plugin.B200FeatureExtractorBackbone(fe, ["s2", "s3", "s4", "s5"], use_checkpoint=True, slide_training=True)

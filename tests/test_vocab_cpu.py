@@ -1,29 +1,45 @@
 """Vocabulary front end (odise_b200/vocab.py): label files / prompts / overlap rule pinned against the reference's own
-functions and data (skipped without /root/reference), the BPE tokenizer checked on a hand-built merge table."""
+functions and data, the BPE tokenizer checked on a hand-built merge table.  The reference's label files are kept under
+tests/golden/openseg_labels/, and digests of what its own functions make of them in tests/golden/ref_pins.pt
+(tools/make_golden_pins.py)."""
+import hashlib
+import json
 import os
 
 import pytest
 import torch
 
 from odise_b200 import vocab
-from oracle import refshim
 
-needs_ref = pytest.mark.skipif(not refshim.available(), reason="/root/reference not present")
-LABELS = "/root/reference/odise/data/datasets/openseg_labels"
+GOLD = os.path.join(os.path.dirname(__file__), "golden")
+LABELS = os.path.join(GOLD, "openseg_labels")
+LABEL_FILES = (("ade20k_150", True), ("coco_panoptic", True), ("ade20k_847", True), ("ade20k_150", False))
+PROMPTS = (None, "a", "photo", "scene")
 
 
-@needs_ref
+def label_file(name, prompt_engineered):
+    return f"{name}_with_prompt_eng.txt" if prompt_engineered else f"{name}.txt"
+
+
+def digest(labels):
+    """SHA-256 of a (nested) list of strings: equal digests <=> equal lists."""
+    return hashlib.sha256(json.dumps(labels).encode()).hexdigest()
+
+
+def _digests():
+    return torch.load(os.path.join(GOLD, "ref_pins.pt"), weights_only=True)["label_digests"]
+
+
 def test_label_files_and_prompts_match_reference():
-    import importlib
-    refshim.install()
-    rb = importlib.import_module("odise.data.build")
+    d = _digests()
     for name, n_cls, n_prompts in (("ade20k_150", 150, 403), ("coco_panoptic", 133, 254), ("ade20k_847", 847, 1342)):
-        mine = vocab.read_label_file(os.path.join(LABELS, f"{name}_with_prompt_eng.txt"))
-        ref = rb.get_openseg_labels(name, prompt_engineered=True)
-        assert mine == ref and len(mine) == n_cls and sum(len(s) for s in mine) == n_prompts     # SURVEY.md §8 K' counts
-        for p in (None, "a", "photo", "scene"):
-            assert vocab.prompt_labels(mine, p) == rb.prompt_labels(ref, p)
-    assert vocab.read_label_file(os.path.join(LABELS, "ade20k_150.txt")) == rb.get_openseg_labels("ade20k_150")
+        f = label_file(name, True)
+        mine = vocab.read_label_file(os.path.join(LABELS, f))
+        assert digest(mine) == d[f] and len(mine) == n_cls and sum(len(s) for s in mine) == n_prompts     # SURVEY.md §8 K' counts
+        for p in PROMPTS:
+            assert digest(vocab.prompt_labels(mine, p)) == d[f"{f}:{p}"], (f, p)
+    f = label_file("ade20k_150", False)
+    assert digest(vocab.read_label_file(os.path.join(LABELS, f))) == d[f]
 
 
 def test_overlap_rule():
@@ -128,21 +144,16 @@ def test_open_state_dict_protocol_swaps_vocabularies():
         bare.load_open_state_dict({"category_head.test_labels": la, "clip_head.test_labels": la})
 
 
-@needs_ref
 def test_prompts_of_the_two_heads_match_reference():
     """ADVICE r1 (high): in the label model the category head scores against the RAW class names (CategoryEmbed
     prompt=None, odise.py:1225; configs/common/models/mask_generator_with_label.py passes none) and only PoolingCLIPHead
-    uses "a photo of a {}." (odise.py:1428).  Pinned on the reference's own defaults and prompt function."""
-    import inspect
-    od = refshim.modules().odise_module
-    assert inspect.signature(od.CategoryEmbed.__init__).parameters["prompt"].default is None
-    assert inspect.signature(od.PoolingCLIPHead.__init__).parameters["prompt"].default == "photo"
-    cfg = open("/root/reference/configs/common/models/mask_generator_with_label.py").read()
-    assert "prompt=" not in cfg.split("category_head=")[1].split("clip_head=")[0]
-    assert "clip_head=L(PoolingCLIPHead)()" in cfg
+    uses "a photo of a {}." (odise.py:1428).  Pinned on the reference's own defaults, config and prompt function."""
+    pins = torch.load(os.path.join(GOLD, "ref_pins.pt"), weights_only=True)
+    assert pins["prompt_defaults"] == {"CategoryEmbed": None, "PoolingCLIPHead": "photo"}
+    assert not pins["label_config"]["category_head_sets_prompt"]
+    assert pins["label_config"]["clip_head_is_default_pooling_clip_head"]
     labels = vocab.read_label_file(os.path.join(LABELS, "ade20k_150_with_prompt_eng.txt"))
     cat, clip, sizes = vocab.vocabulary_prompts(labels)
-    want_cat = od.prompt_labels(labels, inspect.signature(od.CategoryEmbed.__init__).parameters["prompt"].default)
-    want_clip = od.prompt_labels(labels, inspect.signature(od.PoolingCLIPHead.__init__).parameters["prompt"].default)
-    assert cat == [p for s_ in want_cat for p in s_] and clip == [p for s_ in want_clip for p in s_]
+    d = pins["label_digests"]
+    assert digest(cat) == d["odise.prompt_labels:CategoryEmbed"] and digest(clip) == d["odise.prompt_labels:PoolingCLIPHead"]
     assert sizes == [len(s_) for s_ in labels] and len(cat) == len(clip) == 403 and cat != clip

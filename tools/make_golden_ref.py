@@ -14,11 +14,9 @@ import torch
 
 ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..")
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tests"))
 from oracle import cases, refshim  # noqa: E402
 from oracle import ldm as oldm  # noqa: E402
 from oracle import clip as oclip  # noqa: E402
-import test_oracle_cpu as T  # noqa: E402  (reference module constructors)
 
 OUT = os.path.join(ROOT, "tests", "golden")
 h = lambda t: t.detach().clone().to(torch.float32)
@@ -27,12 +25,13 @@ h = lambda t: t.detach().clone().to(torch.float32)
 @torch.no_grad()
 def main():
     assert refshim.available(), "needs /root/reference"
+    torch.set_num_threads(cases.GOLDEN_THREADS)                  # the bits of CPU reductions depend on it
     m = refshim.modules()
     # ---- Mask2Former pixel decoder + ODISE decoder + scoring
     sd, feats, sizes, te, ne = cases.head_case()
-    pd, dec = T._ref_head(m)
-    pd.load_state_dict(T._strip(sd, "sem_seg_head.pixel_decoder."))
-    dec.load_state_dict(T._strip(sd, "sem_seg_head.predictor."))
+    pd, dec = refshim.ref_head(m)
+    pd.load_state_dict(refshim.strip(sd, "sem_seg_head.pixel_decoder."))
+    dec.load_state_dict(refshim.strip(sd, "sem_seg_head.predictor."))
     mf, _, ms = pd.forward_features(feats)
     out = dec(ms, mf)
     logits = m.CategoryODISE.cal_pred_logits(None, dict(mask_embed=out["mask_embed"], text_embed=te, null_embed=ne,
